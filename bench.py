@@ -8,6 +8,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # our arm (one rank per GPU)
     python bench.py --impl reference ...                   # the reference's CPU path, same JSON
+    python bench.py ... --dump-outputs DIR                 # also save the last timed step's logits as DIR/logits.npy
 
 A "step" = one pass of the hot path over one batch.  `value` is measured with the inputs
 resident in HBM; `e2e` goes through the reference-facing predict() call with HOST (pinned)
@@ -449,6 +450,15 @@ def production_shape_block(dev, with_cpu):
     return blk
 
 
+def dump_outputs(out_dir, arrays):
+    """One float32 .npy per output tensor.  Inputs and weights are seeded, so two builds run with the same arguments can be
+    compared array for array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -467,7 +477,14 @@ def main():
     ap.add_argument("--dtype", default="bf16", choices=["bf16", "f32"],
                     help="window dtype: bf16 is the BASELINE workload; f32 (the reference's native dtype) is an extra line")
     ap.add_argument("--tc-splits", type=int, default=3, help="bf16 pieces per fp32 conv1 weight on the tensor cores (3 = fp32-equivalent)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the logits predict() returned in the last timed step to DIR/logits.npy (float32; "
+                         "DIR/logits_rank<r>.npy per rank when N > 1) to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 arm")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -537,6 +554,8 @@ def main():
     total_ms = float(t.item())
     value = world * B * args.steps / (total_ms / 1e3)
     assert torch.isfinite(y).all()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits" if world == 1 else f"logits_rank{rank}": y})
 
     # ---- sustained: >= 3 s of back-to-back steps (the 12 ms headline region is a burst; an issue-bound
     #      kernel scales with the SM clock, which sags under sustained load) -----------------------------

@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -48,3 +50,30 @@ def test_gpu_arm_needs_a_gpu():
         return
     r = _bench("--steps", "1", timeout=120)
     assert r.returncode != 0 and "needs a GPU" in r.stderr
+
+
+def test_argument_checks(tmp_path):
+    r = _bench("--steps", "0", timeout=120)
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+    r = _bench("--impl", "reference", "--dump-outputs", str(tmp_path), timeout=120)
+    assert r.returncode == 2 and "--dump-outputs applies to the b200 arm" in r.stderr
+    assert not os.listdir(tmp_path)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_reproducible(tmp_path):
+    """--dump-outputs writes the last timed step's logits; two runs with the same arguments write the same array."""
+    import numpy as np
+    ys = []
+    for i in range(2):
+        out = tmp_path / str(i)
+        r = _bench("--steps", "2", "--warmup", "3", "--batch", "256", "--sustained-seconds", "0", "--e2e-steps", "1",
+                   "--parity-windows", "0", "--extra-steps", "0", "--no-cpu-baseline", "--dump-outputs", str(out), timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+        assert d["steps"] == 2 and d["n_gpus"] == 1
+        assert os.listdir(out) == ["logits.npy"]
+        y = np.load(out / "logits.npy")
+        assert y.dtype == np.float32 and y.shape == (256,) and np.isfinite(y).all()
+        ys.append(y)
+    assert np.array_equal(ys[0], ys[1])

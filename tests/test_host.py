@@ -2,6 +2,7 @@
 inference, the C-ABI library's exported symbols -- and that the product path fails loudly
 (no CPU fallback) when there is no GPU."""
 import ctypes
+import gzip
 import os
 import re
 
@@ -12,9 +13,7 @@ import torch
 import tskd_b200
 from tskd_b200 import capi
 from tskd_b200.arch import BLOB_KEYS, INERT_KEYS, ArchConfig, arch_from_state_dict
-from conftest import ROOT, load_golden
-
-REF_MODELS = "/root/reference/model"
+from conftest import GOLDEN, ROOT, load_golden
 
 
 def test_library_exports_every_declared_symbol():
@@ -110,10 +109,13 @@ def test_view_contract_rejected():
         tskd_b200.B200MyCNN.from_reference(sd, window=240)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_MODELS), reason="reference checkpoints only exist in the authoring container")
 @pytest.mark.parametrize("n", [2, 3, 4, 5])
-def test_load_legacy_pickles(n):
-    ref = tskd_b200.load_reference_checkpoint(f"{REF_MODELS}/MyCNN{n}.pth")
+def test_load_legacy_pickles(n, tmp_path):
+    """The reference's shipped checkpoints model/MyCNN{n}.pth, stored byte for byte (gzip-compressed) under tests/golden/."""
+    p = tmp_path / f"MyCNN{n}.pth"
+    with gzip.open(os.path.join(GOLDEN, f"MyCNN{n}.pth.gz"), "rb") as f:
+        p.write_bytes(f.read())
+    ref = tskd_b200.load_reference_checkpoint(str(p))
     assert type(ref).__name__ == "PickledMyCNN" and ref.training is False
     m = tskd_b200.B200MyCNN.from_reference(ref)
     g, sd = load_golden("mycnn5_xtestinput.npz" if n == 5 else f"mycnn{n}_ckpt.npz")
